@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- OF-3B training tokens/sec on B200 (BASELINE.json metric), one process per GPU.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path
     python bench.py --impl reference [--steps K] [--warmup W]      # CPU port of the reference (oracle), host cores
 
 Workload (BASELINE.json configs[1], SURVEY.md C2): OF-3B = ViT-L/14 + MPT-1B-shaped LM (HF MptForCausalLM,
@@ -58,7 +58,13 @@ def parse_args():
     ap.add_argument("--micro-batches", type=int, default=1,
                     help="backward passes per optimizer step (the reference's step is LAION + MMC4 = 2, "
                          "train_utils.py:118,172); all but the last run under trainer.no_sync(); tokens/s counts all of them")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (float32): "
+                         "its loss and a fixed seeded sample of the updated fp32 master weights")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 def model_dims(name):
@@ -393,6 +399,29 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+# ----------------------------------------------------------------------------------------------- output dump
+DUMP_SAMPLE = 1 << 22      # sampled weights: 16 MB of float32
+
+
+def dump_outputs(out_dir, loss, bucket, sample=DUMP_SAMPLE, seed=0):
+    """What one training step hands back to its caller: the loss, and the fp32 master weights its AdamW update left.
+    The flat weight buffer holds ~1e9 values at OF-3B, so it is sampled at positions drawn from a fixed seed (the same
+    positions for the same --model); a buffer no larger than `sample` is written whole.
+
+    The step's gradient is not written: a single step reproduces its gradient to ~3e-8 (float atomics), but the
+    training steps before the dump amplify that about tenfold per step, so two runs of the same build differ by ~0.8
+    relative L2 in the last step's gradient against ~2e-3 in the loss and ~6e-4 in the weights (OF-3B, --steps 8,
+    B200 at 1000 W)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"loss": loss.detach().float().reshape(()), "params": bucket.params}
+    if bucket.total > sample:
+        pos = np.sort(np.random.default_rng(seed).choice(bucket.total, size=sample, replace=False))
+        arrays["params"] = bucket.params.index_select(0, torch.from_numpy(pos).to(bucket.device))
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().cpu().numpy().astype(np.float32))
+
+
 # ----------------------------------------------------------------------------------------------- our arm
 def run_ours(args):
     import torch.distributed as dist
@@ -501,8 +530,16 @@ def run_ours(args):
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    ms_total = timed(lambda: run_step(resident), args.steps)
+    last = {}
+
+    def timed_step():
+        last["loss"] = run_step(resident)
+
+    ms_total = timed(timed_step, args.steps)
     clocks = sampler.stop() if rank == 0 else {}
+    if args.dump_outputs and rank == 0:
+        # before anything below runs the step again: the graph's loss buffer and the weights would move on
+        dump_outputs(args.dump_outputs, last["loss"], trainer.bucket)
     ms_step = ms_total / args.steps
     tokens = world * B * T_txt * MB
     # host time needed to ENQUEUE one step (no sync inside): must stay well below ms_step or the GPU starves
