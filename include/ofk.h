@@ -45,8 +45,20 @@ enum {
                                   helpers.py:267-277 (x = branch * gate.tanh() + x), helpers.py:130-131 (Perceiver residuals)   */
   OFK_EPI_DGELU_BF16 = 7,      /* out(bf16) = acc * gelu_erf'(aux(bf16) = z)                 autograd of helpers.py:20           */
   OFK_EPI_BIAS_RESID_F32 = 8,  /* out(f32) = bf16(acc + bias[n]) + aux(f32)  (out may alias aux)  ViT residual adds            */
-  OFK_EPI_BIAS_GELU_BF16 = 9   /* out(bf16) = gelu_erf(acc + bias[n])                        ViT mlp.c_fc + nn.GELU (non-openai) */
+  OFK_EPI_BIAS_GELU_BF16 = 9,  /* out(bf16) = gelu_erf(acc + bias[n])                        ViT mlp.c_fc + nn.GELU (non-openai) */
+  OFK_EPI_SWIGLU_DUAL = 10     /* B = packed [gate; up] weight (OFK_SWIGLU_GROUP layout below), N = 2 * I:
+                                  out(bf16) [M, I] = h = bf16(bf16(silu(g)) * u), g / u = bf16(acc) of the gate / up rows;
+                                  out2(bf16) [M, 2I] = raw bf16(acc) in the packed column order (optional, for the backward).
+                                  A and B K-major only, N % 32 == 0.   HF LlamaMLP: act_fn(gate_proj(x)) * up_proj(x)      */
 };
+
+/* Packed SwiGLU weight: gate_proj and up_proj ([I, D] each, I % 16 == 0) interleaved in groups of OFK_SWIGLU_GROUP rows,
+ *   packed row 32 j + i      = gate row 16 j + i   (i < 16)
+ *   packed row 32 j + 16 + i = up   row 16 j + i
+ * so each 32-column round of the GEMM epilogue holds 16 gate columns and the 16 matching up columns.  The GEMM's raw
+ * output `out2` and the gradient ofk_swiglu_bwd writes use the same column order; a dgrad GEMM of that gradient against
+ * the packed weight gives the gradient of the MLP input in one pass. */
+#define OFK_SWIGLU_GROUP 16
 
 const char* ofk_last_error(void);
 int ofk_abi_version(void);
@@ -121,6 +133,37 @@ int ofk_layernorm_bwd(const void* dy, int dy_is_f32, long long lddy, int rows_pe
                       int group_offset, const float* x, long long ldx, const float* gamma, const float* mean,
                       const float* rstd, int rows, int D, float* dx, long long lddx, const float* dx_add,
                       long long ldadd, float* dgamma, float* dbeta, void* workspace, void* stream);
+
+/* RMSNorm over the last dim, fp32 statistics: y(bf16) = bf16(gamma * (x * rsqrt(mean(x^2) + eps))).  The variant of
+ * the LayerNorm kernels above without centring and without beta.  HF LlamaRMSNorm.forward (input_layernorm /
+ * post_attention_layernorm of LlamaDecoderLayer) followed by the autocast cast in front of the next Linear.
+ *   x: [rows, D] f32 (ldx); y: bf16 (ldy); rstd: [rows] f32 output (may be NULL).  D % 4 == 0, D <= 4096. */
+int ofk_rmsnorm_fwd(const float* x, long long ldx, const float* gamma, float eps, int rows, int D, void* y,
+                    long long ldy, float* rstd, void* stream);
+
+/* RMSNorm backward, input gradient only (frozen gamma): dx(f32) = RMSNorm'(dy) (+ dx_add if non-NULL; may alias dx).
+ * dy: [rows, D] bf16 (dy_is_f32 = 0) or f32.  Autograd of HF LlamaRMSNorm.forward. */
+int ofk_rmsnorm_bwd(const void* dy, int dy_is_f32, long long lddy, const float* x, long long ldx, const float* gamma,
+                    const float* rstd, int rows, int D, float* dx, long long lddx, const float* dx_add, long long ldadd,
+                    void* stream);
+
+/* Rotary position embedding, in place on bf16 rows: x is [batch * T, ldx]; its first nheads * head_dim columns are
+ * nheads heads (q and k of a fused [q | k | v] row: nheads = 2 * heads).  Row r = b * T + t uses
+ * cos / sin[b * cs_bstride + t * head_dim + i] (f32, cs_bstride 0 or T * head_dim).
+ *   inverse = 0: x = bf16(x * cos + rotate_half(x) * sin), products and sum in f32 (HF apply_rotary_pos_emb under
+ *                autocast: bf16 q/k times f32 cos/sin, cast to bf16 by SDPA).
+ *   inverse = 1: the transposed rotation with autograd's rounding (each branch's gradient rounded to bf16, then
+ *                summed): turns dq / dk of the rotated tensors into gradients of the projection outputs.
+ * head_dim % 16 == 0, ldx % 8 == 0, x 16-byte aligned. */
+int ofk_rope(void* x, long long ldx, int batch, int T, int nheads, int head_dim, const float* cos, const float* sin,
+             long long cs_bstride, int inverse, void* stream);
+
+/* SwiGLU backward (autograd of HF LlamaMLP's act_fn(gate_proj(x)) * up_proj(x) under autocast):
+ *   a = bf16(silu(g)),  du = bf16(dh * a),  dg = bf16(bf16(dh * u) * silu'(g))
+ * dh: [rows, I] bf16; gu: [rows, 2I] bf16 packed g / u (out2 of OFK_EPI_SWIGLU_DUAL); dgu: [rows, 2I] bf16 in the same
+ * packed order.  I % 16 == 0, row strides % 8 == 0. */
+int ofk_swiglu_bwd(const void* dh, long long lddh, const void* gu, long long ldgu, int rows, int I, void* dgu,
+                   long long lddgu, void* stream);
 
 /* ------------------------------------------------------------------------------------------------
  * Attention core  O = softmax(scale * Q K^T + mask) V  per (batch, head), head_dim = 64, bf16 in/out,

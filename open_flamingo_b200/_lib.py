@@ -30,6 +30,8 @@ EPI_GATE_RESID_F32 = 6
 EPI_DGELU_BF16 = 7
 EPI_BIAS_RESID_F32 = 8
 EPI_BIAS_GELU_BF16 = 9
+EPI_SWIGLU_DUAL = 10
+SWIGLU_GROUP = 16   # OFK_SWIGLU_GROUP: gate / up rows interleaved in groups of 16 in the packed SwiGLU weight
 
 MASK_NONE = 0
 MASK_MEDIA_EQ = 1
@@ -57,6 +59,11 @@ _SIGNATURES = {
     "ofk_layernorm_bwd": (c_int, [c_void_p, c_int, c_ll, c_int, c_int, c_int, c_void_p, c_ll, c_void_p, c_void_p,
                                   c_void_p, c_int, c_int, c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_void_p,
                                   c_void_p, c_void_p]),
+    "ofk_rmsnorm_fwd": (c_int, [c_void_p, c_ll, c_void_p, c_float, c_int, c_int, c_void_p, c_ll, c_void_p, c_void_p]),
+    "ofk_rmsnorm_bwd": (c_int, [c_void_p, c_int, c_ll, c_void_p, c_ll, c_void_p, c_void_p, c_int, c_int, c_void_p, c_ll,
+                                c_void_p, c_ll, c_void_p]),
+    "ofk_rope": (c_int, [c_void_p, c_ll, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_ll, c_int, c_void_p]),
+    "ofk_swiglu_bwd": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_int, c_int, c_void_p, c_ll, c_void_p]),
     "ofk_attn_fwd": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_int,
                              c_ll, c_ll, c_ll, c_ll, c_ll, c_ll, c_ll, c_ll, c_float, c_int, c_void_p, c_int,
                              c_void_p]),

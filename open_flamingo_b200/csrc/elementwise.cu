@@ -124,6 +124,86 @@ __global__ void __launch_bounds__(256) gate_bwd_kernel(const float* __restrict__
   }
 }
 
+// ---- rotary position embedding (HF apply_rotary_pos_emb), in place on the q / k heads of fused bf16 rows.
+// One thread per (row, head, 8-column chunk of the head's first half): it owns columns i and i + hd/2, the pair
+// rotate_half mixes.  __fmul_rn / __fadd_rn keep the products and the sum separately rounded, as torch computes them.
+__device__ __forceinline__ void load8f(const float* p, float (&v)[8]) {
+  const float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + 4);
+  v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
+}
+__device__ __forceinline__ void unpack8(uint4 u, float (&v)[8]) {
+  v[0] = bf16_lo(u.x); v[1] = bf16_hi(u.x); v[2] = bf16_lo(u.y); v[3] = bf16_hi(u.y);
+  v[4] = bf16_lo(u.z); v[5] = bf16_hi(u.z); v[6] = bf16_lo(u.w); v[7] = bf16_hi(u.w);
+}
+__device__ __forceinline__ uint4 pack8(const float (&v)[8]) {
+  return make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+}
+
+__global__ void __launch_bounds__(256) rope_kernel(__nv_bfloat16* __restrict__ x, long long ldx, int T, int nheads, int hd,
+                                                   const float* __restrict__ cosp, const float* __restrict__ sinp,
+                                                   long long csb, int inverse, long long total) {
+  const int chunks = hd / 16;
+  const int half = hd / 2;
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
+    const int c = (int)(idx % chunks);
+    const long long rh = idx / chunks;
+    const int h = (int)(rh % nheads);
+    const long long r = rh / nheads;
+    const long long b = r / T, t = r % T;
+    const int i0 = c * 8;
+    __nv_bfloat16* p = x + r * ldx + (long long)h * hd + i0;
+    const float* cs = cosp + b * csb + t * hd + i0;
+    const float* sn = sinp + b * csb + t * hd + i0;
+    float lo[8], hi[8], cl[8], ch[8], sl[8], sh[8];
+    unpack8(*reinterpret_cast<const uint4*>(p), lo);
+    unpack8(*reinterpret_cast<const uint4*>(p + half), hi);
+    load8f(cs, cl); load8f(cs + half, ch); load8f(sn, sl); load8f(sn + half, sh);
+    float olo[8], ohi[8];
+    if (!inverse) {
+      // out = x * cos + rotate_half(x) * sin,  rotate_half(x) = (-x_hi, x_lo)
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        olo[i] = __fsub_rn(__fmul_rn(lo[i], cl[i]), __fmul_rn(hi[i], sl[i]));
+        ohi[i] = __fadd_rn(__fmul_rn(hi[i], ch[i]), __fmul_rn(lo[i], sh[i]));
+      }
+    } else {
+      // autograd: dx = bf16(d * cos) + rotate_half^T(bf16(d * sin)),  rotate_half^T(y) = (y_hi, -y_lo)
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        olo[i] = bf16_round(lo[i] * cl[i]) + bf16_round(hi[i] * sh[i]);
+        ohi[i] = bf16_round(hi[i] * ch[i]) - bf16_round(lo[i] * sl[i]);
+      }
+    }
+    *reinterpret_cast<uint4*>(p) = pack8(olo);
+    *reinterpret_cast<uint4*>(p + half) = pack8(ohi);
+  }
+}
+
+// ---- SwiGLU backward on the packed [g | u] layout (OFK_SWIGLU_GROUP): one thread per 8 h columns of one row.
+__global__ void __launch_bounds__(256) swiglu_bwd_kernel(const __nv_bfloat16* __restrict__ dh, long long lddh,
+                                                         const __nv_bfloat16* __restrict__ gu, long long ldgu, int I,
+                                                         __nv_bfloat16* __restrict__ dgu, long long lddgu, long long total) {
+  const int per_row = I / 8;
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
+    const long long r = idx / per_row;
+    const int j8 = (int)(idx % per_row) * 8;                               // first h column
+    const int pc = (j8 / OFK_SWIGLU_GROUP) * 2 * OFK_SWIGLU_GROUP + j8 % OFK_SWIGLU_GROUP;   // its gate column
+    float d[8], g[8], u[8], dg[8], du[8];
+    unpack8(*reinterpret_cast<const uint4*>(dh + r * lddh + j8), d);
+    unpack8(*reinterpret_cast<const uint4*>(gu + r * ldgu + pc), g);
+    unpack8(*reinterpret_cast<const uint4*>(gu + r * ldgu + pc + OFK_SWIGLU_GROUP), u);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      du[i] = d[i] * bf16_round(silu(g[i]));
+      dg[i] = bf16_round(d[i] * u[i]) * silu_grad(g[i]);
+    }
+    *reinterpret_cast<uint4*>(dgu + r * lddgu + pc) = pack8(dg);
+    *reinterpret_cast<uint4*>(dgu + r * lddgu + pc + OFK_SWIGLU_GROUP) = pack8(du);
+  }
+}
+
 __global__ void add_f32_kernel(float* __restrict__ dst, const float* __restrict__ src, long long n) {
   const long long n4 = n / 4;
   const long long stride = (long long)gridDim.x * blockDim.x;
@@ -274,6 +354,37 @@ extern "C" int ofk_gate_bwd(const float* dout, const void* branch, const float* 
   if (n % 8 != 0) return ofk_set_error(OFK_ERR_ARG, "gate_bwd: n must be a multiple of 8");
   gate_bwd_kernel<<<grid_for(n / 8, 256), 256, 0, (cudaStream_t)stream>>>(dout, (const __nv_bfloat16*)branch, gate,
                                                                            (__nv_bfloat16*)dbranch, dgate, n);
+  OFK_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int ofk_rope(void* x, long long ldx, int batch, int T, int nheads, int head_dim, const float* cos,
+                        const float* sin, long long cs_bstride, int inverse, void* stream) {
+  if (!x || !cos || !sin) return ofk_set_error(OFK_ERR_ARG, "rope: null pointer");
+  if (batch <= 0 || T <= 0 || nheads <= 0) return 0;
+  if (head_dim <= 0 || head_dim % 16 != 0 || ldx < (long long)nheads * head_dim)
+    return ofk_set_error(OFK_ERR_ARG, "rope: head_dim must be a multiple of 16 and the heads must fit the row");
+  if ((reinterpret_cast<uintptr_t>(x) & 15) || ldx % 8 != 0 || (reinterpret_cast<uintptr_t>(cos) & 15) ||
+      (reinterpret_cast<uintptr_t>(sin) & 15) || cs_bstride % 4 != 0)
+    return ofk_set_error(OFK_ERR_ALIGN, "rope: x / cos / sin must be 16-byte aligned with 16-byte row strides");
+  const long long total = (long long)batch * T * nheads * (head_dim / 16);
+  rope_kernel<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>((__nv_bfloat16*)x, ldx, T, nheads, head_dim, cos,
+                                                                      sin, cs_bstride, inverse, total);
+  OFK_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int ofk_swiglu_bwd(const void* dh, long long lddh, const void* gu, long long ldgu, int rows, int I, void* dgu,
+                              long long lddgu, void* stream) {
+  if (!dh || !gu || !dgu) return ofk_set_error(OFK_ERR_ARG, "swiglu_bwd: null pointer");
+  if (rows <= 0) return 0;
+  if (I <= 0 || I % OFK_SWIGLU_GROUP != 0) return ofk_set_error(OFK_ERR_ARG, "swiglu_bwd: I must be a multiple of 16");
+  if ((reinterpret_cast<uintptr_t>(dh) & 15) || (reinterpret_cast<uintptr_t>(gu) & 15) ||
+      (reinterpret_cast<uintptr_t>(dgu) & 15) || lddh % 8 != 0 || ldgu % 8 != 0 || lddgu % 8 != 0)
+    return ofk_set_error(OFK_ERR_ALIGN, "swiglu_bwd: operands must be 16-byte aligned with 16-byte row strides");
+  const long long total = (long long)rows * (I / 8);
+  swiglu_bwd_kernel<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>(
+      (const __nv_bfloat16*)dh, lddh, (const __nv_bfloat16*)gu, ldgu, I, (__nv_bfloat16*)dgu, lddgu, total);
   OFK_CHECK_LAUNCH();
   return 0;
 }

@@ -229,6 +229,30 @@ __device__ __forceinline__ void aux_commit(uint32_t stage, const uint4 (&pre)[EL
   __syncwarp();
 }
 
+// Store a 32-row x 16-column bf16 tile (lane's row in `w`) coalesced: two 16-byte pieces per row, 16 rows per
+// instruction.  The SwiGLU epilogue's `h` output: one 32-column accumulator round yields 16 columns of h.
+__device__ __forceinline__ void warp_store_tile16_bf16(uint32_t stage, const uint32_t (&w)[8], void* gbase, long long ld,
+                                                       int row0, int col0, int M, int N, int streaming) {
+  const int lane = threadIdx.x & 31;
+  st_shared_v4(stage + stage_off(lane, 0), make_uint4(w[0], w[1], w[2], w[3]));
+  st_shared_v4(stage + stage_off(lane, 1), make_uint4(w[4], w[5], w[6], w[7]));
+  __syncwarp();
+  const int piece = lane & 1, rsub = lane >> 1;
+  const int col = col0 + piece * 8;
+#pragma unroll
+  for (int it = 0; it < 2; ++it) {
+    const int r = it * 16 + rsub;
+    const uint4 v = ld_shared_v4(stage + stage_off(r, piece));
+    const int row = row0 + r;
+    if (row < M && col < N) {
+      void* g = reinterpret_cast<__nv_bfloat16*>(gbase) + (long long)row * ld + col;
+      if (streaming) st_global_cs_v4(g, v);
+      else *reinterpret_cast<uint4*>(g) = v;
+    }
+  }
+  __syncwarp();
+}
+
 template <int EPI>
 struct AuxBytes { static constexpr int value = (EPI == OFK_EPI_GATE_RESID_F32 || EPI == OFK_EPI_BIAS_RESID_F32) ? 4 : (EPI == OFK_EPI_DGELU_BF16 ? 2 : 0); };
 
@@ -309,6 +333,21 @@ __device__ __forceinline__ void epilogue32(const GemmParams& p, float gate_t, ui
     }
     pack32_bf16(v, w);
     warp_store_tile<2, 0>(stage, w, p.out, p.ldo, row0, col0, p.M, p.N, p.stream_out, p.out_rpg, p.out_gs, p.out_go);
+  } else if constexpr (EPI == OFK_EPI_SWIGLU_DUAL) {
+    // columns [col0, col0+16) are gate rows, [col0+16, col0+32) the matching up rows (OFK_SWIGLU_GROUP packing):
+    // h = bf16(bf16(silu(g)) * u) for the 16 columns [col0/2, col0/2+16) of out, as HF LlamaMLP under autocast
+#pragma unroll
+    for (int i = 0; i < 32; ++i) v[i] = bf16_round(v[i]);
+    if (p.out2 != nullptr) {
+      uint32_t wgu[16];
+      pack32_bf16(v, wgu);
+      warp_store_tile<2, 0>(stage, wgu, p.out2, p.ldo2, row0, col0, p.M, p.N, p.stream_out);
+    }
+    uint32_t wh[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+      wh[i] = pack_bf16x2(bf16_round(silu(v[2 * i])) * v[16 + 2 * i], bf16_round(silu(v[2 * i + 1])) * v[17 + 2 * i]);
+    warp_store_tile16_bf16(stage, wh, p.out, p.ldo, row0, col0 / 2, p.M, p.N / 2, p.stream_out);
   }
 }
 
@@ -879,6 +918,7 @@ static int dispatch_epi2(int epi, int a_mn, int b_mn, const CUtensorMap& ta, con
     case OFK_EPI_DGELU_BF16: return dispatch_major2<OFK_EPI_DGELU_BF16>(a_mn, b_mn, ta, tb, p, s);
     case OFK_EPI_BIAS_RESID_F32: return dispatch_major2<OFK_EPI_BIAS_RESID_F32>(a_mn, b_mn, ta, tb, p, s);
     case OFK_EPI_BIAS_GELU_BF16: return dispatch_major2<OFK_EPI_BIAS_GELU_BF16>(a_mn, b_mn, ta, tb, p, s);
+    case OFK_EPI_SWIGLU_DUAL: return launch2<0, 0, OFK_EPI_SWIGLU_DUAL>(ta, tb, p, s);   // K-major only (gemm_impl)
   }
   return ofk_set_error(OFK_ERR_ARG, "unknown GEMM epilogue");
 }
@@ -906,6 +946,7 @@ static int dispatch_epi(int epi, int a_mn, int b_mn, const CUtensorMap& ta, cons
     case OFK_EPI_DGELU_BF16: return dispatch_major<BN, OFK_EPI_DGELU_BF16>(a_mn, b_mn, ta, tb, p, s);
     case OFK_EPI_BIAS_RESID_F32: return dispatch_major<BN, OFK_EPI_BIAS_RESID_F32>(a_mn, b_mn, ta, tb, p, s);
     case OFK_EPI_BIAS_GELU_BF16: return dispatch_major<BN, OFK_EPI_BIAS_GELU_BF16>(a_mn, b_mn, ta, tb, p, s);
+    case OFK_EPI_SWIGLU_DUAL: return launch<BN, 0, 0, OFK_EPI_SWIGLU_DUAL>(ta, tb, p, s);
   }
   return ofk_set_error(OFK_ERR_ARG, "unknown GEMM epilogue");
 }
@@ -951,6 +992,8 @@ static int gemm_impl(int epi, int a_mn_major, int b_mn_major, const void* A, lon
   if ((epi == OFK_EPI_GATE_RESID_F32 || epi == OFK_EPI_BIAS_RESID_F32 || epi == OFK_EPI_DGELU_BF16) && !aux)
     return ofk_set_error(OFK_ERR_ARG, "epilogue needs aux operand");
   if (epi == OFK_EPI_GELU_DUAL && !out2) return ofk_set_error(OFK_ERR_ARG, "GELU_DUAL needs out2");
+  if (epi == OFK_EPI_SWIGLU_DUAL && (a_mn_major || b_mn_major || N % (2 * OFK_SWIGLU_GROUP) != 0 || splits > 1 || out_rpg > 0))
+    return ofk_set_error(OFK_ERR_ARG, "SWIGLU_DUAL needs K-major A and B, N % 32 == 0 and no split-K");
   if (g_num_sms == 0) {
     int dev = 0;
     cudaGetDevice(&dev);

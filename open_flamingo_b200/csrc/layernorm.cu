@@ -5,6 +5,7 @@
 // they are the TMA-ready A operand of the following GEMM (the reference's autocast casts the fp32 LN
 // output to bf16 inside nn.Linear -- same rounding point), and can write them at an offset/stride so the
 // two LayerNorms of PerceiverAttention fill cat((x, latents), -2) (helpers.py:53) without a copy kernel.
+// RMS = true is the RMSNorm variant (HF LlamaRMSNorm: no centring, no beta, y = gamma * (x * rstd)).
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -20,7 +21,7 @@ __device__ __forceinline__ long long map_row(int r, int rpg, int gstride, int go
 }
 
 // One warp per row; each lane keeps NV float4 (columns (i*32 + lane)*4) in registers.
-template <int NV>
+template <int NV, bool RMS = false>
 __global__ void __launch_bounds__(128) ln_fwd_kernel(const float* __restrict__ x, long long ldx,
                                                      const float* __restrict__ gamma, const float* __restrict__ beta,
                                                      float eps, int rows, int D, void* __restrict__ y, int y_is_f32,
@@ -42,7 +43,7 @@ __global__ void __launch_bounds__(128) ln_fwd_kernel(const float* __restrict__ x
       v[i] = make_float4(0.f, 0.f, 0.f, 0.f);
     }
   }
-  const float mean = warp_sum(s) / (float)D;
+  const float mean = RMS ? 0.f : warp_sum(s) / (float)D;
   float sq = 0.f;
 #pragma unroll
   for (int i = 0; i < NV; ++i) {
@@ -54,7 +55,7 @@ __global__ void __launch_bounds__(128) ln_fwd_kernel(const float* __restrict__ x
   }
   const float rstd = rsqrtf(warp_sum(sq) / (float)D + eps);
   if (lane == 0) {
-    if (mean_out) mean_out[row] = mean;
+    if (!RMS && mean_out) mean_out[row] = mean;
     if (rstd_out) rstd_out[row] = rstd;
   }
   const long long orow = map_row(row, rpg, gstride, goff);
@@ -63,9 +64,14 @@ __global__ void __launch_bounds__(128) ln_fwd_kernel(const float* __restrict__ x
     const int c = (i * 32 + lane) * 4;
     if (c < D) {
       const float4 g = __ldg(reinterpret_cast<const float4*>(gamma + c));
-      const float4 b = __ldg(reinterpret_cast<const float4*>(beta + c));
-      const float o0 = (v[i].x - mean) * rstd * g.x + b.x, o1 = (v[i].y - mean) * rstd * g.y + b.y;
-      const float o2 = (v[i].z - mean) * rstd * g.z + b.z, o3 = (v[i].w - mean) * rstd * g.w + b.w;
+      float o0, o1, o2, o3;
+      if constexpr (RMS) {
+        o0 = (v[i].x * rstd) * g.x; o1 = (v[i].y * rstd) * g.y; o2 = (v[i].z * rstd) * g.z; o3 = (v[i].w * rstd) * g.w;
+      } else {
+        const float4 b = __ldg(reinterpret_cast<const float4*>(beta + c));
+        o0 = (v[i].x - mean) * rstd * g.x + b.x; o1 = (v[i].y - mean) * rstd * g.y + b.y;
+        o2 = (v[i].z - mean) * rstd * g.z + b.z; o3 = (v[i].w - mean) * rstd * g.w + b.w;
+      }
       if (y_is_f32) {
         *reinterpret_cast<float4*>(reinterpret_cast<float*>(y) + orow * ldy + c) = make_float4(o0, o1, o2, o3);
       } else {
@@ -81,7 +87,7 @@ __global__ void __launch_bounds__(128) ln_fwd_kernel(const float* __restrict__ x
 constexpr int LNB_THREADS = 256;
 constexpr int LNB_MAX_BLOCKS = 592;  // 148 SMs x 4 resident blocks
 
-template <int G>
+template <int G, bool RMS = false>
 __global__ void __launch_bounds__(LNB_THREADS) ln_bwd_kernel(
     const void* __restrict__ dy, int dy_is_f32, long long lddy, int rpg, int gstride, int goff,
     const float* __restrict__ x, long long ldx, const float* __restrict__ gamma, const float* __restrict__ mean,
@@ -100,7 +106,7 @@ __global__ void __launch_bounds__(LNB_THREADS) ln_bwd_kernel(
   const float invD = 1.0f / (float)D;
   int par = 0;
   for (int r = blockIdx.x; r < rows; r += gridDim.x) {
-    const float mu = mean[r], rs = rstd[r];
+    const float mu = RMS ? 0.f : mean[r], rs = rstd[r];
     const long long yr = map_row(r, rpg, gstride, goff);
     float4 xh[G], dyv[G];
     float s1 = 0.f, s2 = 0.f;
@@ -124,6 +130,7 @@ __global__ void __launch_bounds__(LNB_THREADS) ln_bwd_kernel(
         dyv[g] = make_float4(0.f, 0.f, 0.f, 0.f);
       }
     }
+    if constexpr (RMS) s1 = 0.f;   // no centring: the mean(dy * gamma) term drops out
     s1 = warp_sum(s1); s2 = warp_sum(s2);
     if (lane == 0) { s_red[par][warp][0] = s1; s_red[par][warp][1] = s2; }
     __syncthreads();
@@ -245,5 +252,45 @@ extern "C" int ofk_layernorm_bwd(const void* dy, int dy_is_f32, long long lddy, 
     ln_bwd_reduce_kernel<<<dim3((2 * D + 63) / 64, nblocks >= 64 ? LNR_CHUNKS : 1), 256, 0, s>>>(part, nblocks, D, dgamma, dbeta);
     OFK_CHECK_LAUNCH();
   }
+  return 0;
+}
+
+extern "C" int ofk_rmsnorm_fwd(const float* x, long long ldx, const float* gamma, float eps, int rows, int D, void* y,
+                               long long ldy, float* rstd, void* stream_) {
+  using namespace ofk;
+  if (!x || !gamma || !y) return ofk_set_error(OFK_ERR_ARG, "rmsnorm: null pointer");
+  if (rows <= 0) return 0;
+  if (D <= 0 || D % 4 != 0 || D > 4096) return ofk_set_error(OFK_ERR_ARG, "rmsnorm: D must be a multiple of 4, <= 4096");
+  if (ldx % 4 != 0 || ldy % 4 != 0) return ofk_set_error(OFK_ERR_ALIGN, "rmsnorm: row strides must be multiples of 4");
+  cudaStream_t s = (cudaStream_t)stream_;
+  const int grid = (rows + 3) / 4;
+  if (D <= 1024)
+    ln_fwd_kernel<8, true><<<grid, 128, 0, s>>>(x, ldx, gamma, nullptr, eps, rows, D, y, 0, ldy, 0, 0, 0, nullptr, rstd);
+  else if (D <= 2048)
+    ln_fwd_kernel<16, true><<<grid, 128, 0, s>>>(x, ldx, gamma, nullptr, eps, rows, D, y, 0, ldy, 0, 0, 0, nullptr, rstd);
+  else
+    ln_fwd_kernel<32, true><<<grid, 128, 0, s>>>(x, ldx, gamma, nullptr, eps, rows, D, y, 0, ldy, 0, 0, 0, nullptr, rstd);
+  OFK_CHECK_LAUNCH();
+  return 0;
+}
+
+extern "C" int ofk_rmsnorm_bwd(const void* dy, int dy_is_f32, long long lddy, const float* x, long long ldx,
+                               const float* gamma, const float* rstd, int rows, int D, float* dx, long long lddx,
+                               const float* dx_add, long long ldadd, void* stream_) {
+  using namespace ofk;
+  if (!dy || !x || !gamma || !rstd || !dx) return ofk_set_error(OFK_ERR_ARG, "rmsnorm bwd: null pointer");
+  if (rows <= 0) return 0;
+  if (D <= 0 || D % 4 != 0 || D > 4096) return ofk_set_error(OFK_ERR_ARG, "rmsnorm bwd: D must be a multiple of 4, <= 4096");
+  if (ldx % 4 != 0 || lddy % 4 != 0 || lddx % 4 != 0 || (dx_add && ldadd % 4 != 0))
+    return ofk_set_error(OFK_ERR_ALIGN, "rmsnorm bwd: row strides must be multiples of 4");
+  cudaStream_t s = (cudaStream_t)stream_;
+  const int nblocks = rows < LNB_MAX_BLOCKS ? rows : LNB_MAX_BLOCKS;
+  if (D <= 1024)
+    ln_bwd_kernel<1, true><<<nblocks, LNB_THREADS, 0, s>>>(dy, dy_is_f32, lddy, 0, 0, 0, x, ldx, gamma, nullptr, rstd, rows, D, dx, lddx, dx_add, ldadd, nullptr);
+  else if (D <= 2048)
+    ln_bwd_kernel<2, true><<<nblocks, LNB_THREADS, 0, s>>>(dy, dy_is_f32, lddy, 0, 0, 0, x, ldx, gamma, nullptr, rstd, rows, D, dx, lddx, dx_add, ldadd, nullptr);
+  else
+    ln_bwd_kernel<4, true><<<nblocks, LNB_THREADS, 0, s>>>(dy, dy_is_f32, lddy, 0, 0, 0, x, ldx, gamma, nullptr, rstd, rows, D, dx, lddx, dx_add, ldadd, nullptr);
+  OFK_CHECK_LAUNCH();
   return 0;
 }

@@ -255,6 +255,13 @@ __device__ __forceinline__ float gelu_exact_grad(float x) {
 __device__ __forceinline__ float quick_gelu(float x) {
   return x * rcp_approx(1.0f + ex2_approx(-1.702f * 1.4426950408889634f * x));
 }
+// SiLU (HF LlamaMLP act_fn) and its derivative; the MUFU sigmoid is a few fp32 ulp off, far below bf16 resolution
+__device__ __forceinline__ float sigmoid_approx(float x) { return rcp_approx(1.0f + ex2_approx(-1.4426950408889634f * x)); }
+__device__ __forceinline__ float silu(float x) { return x * sigmoid_approx(x); }
+__device__ __forceinline__ float silu_grad(float x) {
+  const float s = sigmoid_approx(x);
+  return s * fmaf(x, 1.0f - s, 1.0f);
+}
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -407,3 +407,91 @@ def gemm_grouped(a, b, *, a_mn=False, b_mn=False, epi=L.EPI_STORE_BF16, out, M, 
         out.data_ptr(), out.stride(0), L.ptr(bias), out_map[0], out_map[1], out_map[2], ak_map[0], ak_map[1], ak_map[2],
         L.stream_ptr()))
     return out
+
+
+def rmsnorm_fwd(x, gamma, eps):
+    """x: [rows, D] f32.  Returns (y bf16, rstd f32 [rows])."""
+    L.require_cuda(x, gamma)
+    _rowmajor_2d(x, "x")
+    if x.dtype != f32 or gamma.dtype != f32 or not gamma.is_contiguous() or gamma.numel() != x.shape[1]:
+        raise ValueError("rmsnorm expects float32 x [rows, D] and a contiguous float32 gamma [D]")
+    rows, D = x.shape
+    y = torch.empty((rows, D), device=x.device, dtype=bf16)
+    rstd = torch.empty(rows, device=x.device, dtype=f32)
+    L.check(L.lib().ofk_rmsnorm_fwd(x.data_ptr(), x.stride(0), gamma.data_ptr(), eps, rows, D, y.data_ptr(), y.stride(0),
+                                    rstd.data_ptr(), L.stream_ptr()))
+    return y, rstd
+
+
+def rmsnorm_bwd(dy, x, gamma, rstd, *, dx_add=None):
+    """dx(f32) = RMSNorm'(dy) (+ dx_add).  dy bf16 or f32 [rows, D]; gamma frozen (no dgamma)."""
+    L.require_cuda(dy, x, gamma, rstd, dx_add)
+    _rowmajor_2d(dy, "dy")
+    _rowmajor_2d(x, "x")
+    if dy.shape != x.shape or x.dtype != f32 or dy.dtype not in (bf16, f32):
+        raise ValueError("rmsnorm_bwd: dy (bf16/f32) and x (f32) must share the shape [rows, D]")
+    if dx_add is not None:
+        _rowmajor_2d(dx_add, "dx_add")
+        if dx_add.dtype != f32 or dx_add.shape != x.shape:
+            raise ValueError("rmsnorm_bwd: dx_add must be float32 like x")
+    rows, D = x.shape
+    dx = torch.empty((rows, D), device=x.device, dtype=f32)
+    L.check(L.lib().ofk_rmsnorm_bwd(dy.data_ptr(), int(dy.dtype == f32), dy.stride(0), x.data_ptr(), x.stride(0),
+                                    gamma.data_ptr(), rstd.data_ptr(), rows, D, dx.data_ptr(), dx.stride(0),
+                                    L.ptr(dx_add), 0 if dx_add is None else dx_add.stride(0), L.stream_ptr()))
+    return dx
+
+
+def rope_(x, batch, T, nheads, head_dim, cos, sin, *, inverse=False):
+    """In place on x [batch*T, ld] bf16: rotate the first nheads heads of every row (HF apply_rotary_pos_emb;
+    inverse=True applies its transpose, for the backward).  cos / sin: f32 [1 or batch, T, head_dim]."""
+    L.require_cuda(x, cos, sin)
+    _rowmajor_2d(x, "x")
+    if x.dtype != bf16 or x.shape[0] != batch * T or x.shape[1] < nheads * head_dim:
+        raise ValueError(f"rope: x must be bf16 [{batch * T}, >= {nheads * head_dim}], got {tuple(x.shape)} {x.dtype}")
+    for t, name in ((cos, "cos"), (sin, "sin")):
+        if t.dtype != f32 or t.dim() != 3 or t.shape[0] not in (1, batch) or tuple(t.shape[1:]) != (T, head_dim) \
+                or not t.is_contiguous():
+            raise ValueError(f"rope: {name} must be a contiguous float32 [1 or {batch}, {T}, {head_dim}] tensor")
+    if cos.shape != sin.shape:
+        raise ValueError("rope: cos and sin shapes differ")
+    cs_bstride = 0 if cos.shape[0] == 1 else T * head_dim
+    L.check(L.lib().ofk_rope(x.data_ptr(), x.stride(0), batch, T, nheads, head_dim, cos.data_ptr(), sin.data_ptr(),
+                             cs_bstride, int(bool(inverse)), L.stream_ptr()))
+    return x
+
+
+def swiglu_gemm(x, w_packed, *, want_gu=True):
+    """h = bf16(silu(g)) * u for the packed [gate; up] weight (OFK_EPI_SWIGLU_DUAL).  x: [R, D] bf16,
+    w_packed: [2I, D] bf16.  Returns (h [R, I], gu [R, 2I] packed raw projections or None)."""
+    L.require_cuda(x, w_packed)
+    _rowmajor_2d(x, "x")
+    _rowmajor_2d(w_packed, "w_packed")
+    if x.dtype != bf16 or w_packed.dtype != bf16:
+        raise ValueError("swiglu_gemm operands must be bfloat16")
+    R, K = x.shape
+    N = w_packed.shape[0]
+    if w_packed.shape[1] != K or N % (2 * L.SWIGLU_GROUP) != 0:
+        raise ValueError(f"swiglu_gemm: w_packed must be [2I, {K}] with I % {L.SWIGLU_GROUP} == 0, got {tuple(w_packed.shape)}")
+    h = torch.empty((R, N // 2), device=x.device, dtype=bf16)
+    gu = torch.empty((R, N), device=x.device, dtype=bf16) if want_gu else None
+    ws = _gemm_workspace(x.device) if (R >= 512 and N >= 256 and K >= 3072 and not _comm_in_flight) else None
+    L.check(L.lib().ofk_gemm_bf16_ws(
+        L.EPI_SWIGLU_DUAL, 0, 0, x.data_ptr(), x.stride(0), w_packed.data_ptr(), w_packed.stride(0), R, N, K, 1, 0,
+        h.data_ptr(), h.stride(0), L.ptr(gu), 0 if gu is None else gu.stride(0), 0, 0, 0, 0,
+        L.ptr(ws), 0 if ws is None else ws.numel(), L.stream_ptr()))
+    return h, gu
+
+
+def swiglu_bwd(dh, gu):
+    """dh: [R, I] bf16, gu: [R, 2I] packed bf16 g / u.  Returns dgu [R, 2I] bf16 in the packed order."""
+    L.require_cuda(dh, gu)
+    _rowmajor_2d(dh, "dh")
+    _rowmajor_2d(gu, "gu")
+    R, I = dh.shape
+    if dh.dtype != bf16 or gu.dtype != bf16 or tuple(gu.shape) != (R, 2 * I):
+        raise ValueError("swiglu_bwd: dh [R, I] and gu [R, 2I] must be bfloat16")
+    dgu = torch.empty((R, 2 * I), device=dh.device, dtype=bf16)
+    L.check(L.lib().ofk_swiglu_bwd(dh.data_ptr(), dh.stride(0), gu.data_ptr(), gu.stride(0), R, I, dgu.data_ptr(),
+                                   dgu.stride(0), L.stream_ptr()))
+    return dgu

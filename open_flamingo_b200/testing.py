@@ -1,5 +1,5 @@
 """Offline construction helpers (no hub / no open_clip): a tokenizer-like object and random-init model builders
-with the OF-3B / OF-9B shapes.  Used by tests, __graft_entry__.smoke() and bench.py."""
+with the OF-3B / OF-9B shapes (MPT, and LLaMA for the first OF-9B release).  Used by tests, __graft_entry__.smoke() and bench.py."""
 import torch
 
 from .src.factory import create_model_and_transforms
@@ -56,14 +56,32 @@ def build_mpt(mpt_kw, dtype=torch.float32, device="cpu", seed=0):
     return lm.to(dtype).eval()
 
 
+# LLaMA-7B, the language model of the first OpenFlamingo-9B release
+LLAMA_7B = dict(hidden_size=4096, num_hidden_layers=32, num_attention_heads=32, num_key_value_heads=32,
+                intermediate_size=11008, vocab_size=32000)
+
+
+def build_llama(llama_kw, dtype=torch.float32, device="cpu", seed=0):
+    """Random-init HF LlamaForCausalLM with the given LlamaConfig fields (SDPA attention, HF's default)."""
+    from transformers import LlamaConfig, LlamaForCausalLM
+    torch.manual_seed(seed)
+    cfg = LlamaConfig(**llama_kw)
+    cfg._attn_implementation = "sdpa"
+    with torch.device(device):
+        lm = LlamaForCausalLM(cfg)
+    return lm.to(dtype).eval()
+
+
 def build_flamingo(vit_cfg, mpt_kw, cross_attn_every_n_layers=1, device="cuda", freeze_lm_embeddings=True, seed=0,
-                   lm_dtype=torch.float32, gate_init=None):
+                   lm_dtype=torch.float32, gate_init=None, lm_builder=build_mpt):
     """Random-init Flamingo through the public factory.  gate_init: None keeps the reference's zero gates
-    (helpers.py:255,258); a float f draws gates ~ U(-f, f) so the gated path is actually exercised."""
+    (helpers.py:255,258); a float f draws gates ~ U(-f, f) so the gated path is actually exercised.
+    lm_builder(mpt_kw, dtype=, device=, seed=) makes the language model: build_mpt (default) or build_llama, with
+    `mpt_kw` the matching config fields."""
     torch.manual_seed(seed)
     with torch.device(device):
         vit = VisionTransformer(**vit_cfg)
-    lm = build_mpt(mpt_kw, dtype=lm_dtype, device=device, seed=seed + 1)
+    lm = lm_builder(mpt_kw, dtype=lm_dtype, device=device, seed=seed + 1)
     base_vocab = mpt_kw["vocab_size"]
     tok = SimpleTokenizer(base_vocab)
     model, image_processor, tok = create_model_and_transforms(
